@@ -61,7 +61,32 @@ def parse_args():
     p.add_argument("--no-sweep", action="store_true", help="skip the queue-count sweep (1..1024 request queues)")
     p.add_argument("--no-mirror", action="store_true", help="skip the mirrored-bdev leg (config 5; runs when --gpus >= 2)")
     p.add_argument("--no-extra", action="store_true", help="skip the 4 KiB random-write / 128 KiB sequential-read legs")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps of the headline leg, write what its last step returned (completion fields "
+                        "and read payload of a fixed sample of requests) as DIR/<name>.npy, for comparing two builds")
     return p.parse_args()
+
+
+DUMP_REQUESTS = 2048           # 2048 x 4 KiB of payload as float32 = 32 MiB
+
+
+def dump_outputs(out_dir: str, prefix: str, t: traces.Trace, arena, cpls: np.ndarray, torch) -> None:
+    """What a caller of a single-element-SG leg receives after its last step, for a fixed, seeded sample of its requests:
+    the completion fields the reference defines plus data_transferred, and each request's client buffer (`arena`, a
+    CUDA tensor).  Values are exact in float64 (completion fields) and float32 (bytes)."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(t.reqs)
+    assert len(t.iovs) == n, "one SG element per request"
+    idx = np.sort(np.random.default_rng(0xD0).choice(n, size=min(n, DUMP_REQUESTS), replace=False))
+    buf = t.iovs[idx]
+    ln = int(buf["len"][0])
+    assert (buf["len"] == ln).all()
+    off = torch.from_numpy(buf["addr"].astype(np.int64)).to(arena.device)
+    payload = arena[off[:, None] + torch.arange(ln, device=arena.device)[None, :]].cpu().numpy()
+    np.save(os.path.join(out_dir, f"{prefix}_request_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, f"{prefix}_payload.npy"), payload.astype(np.float32))
+    for f in abi.CPL_PARITY_FIELDS + ("data_transferred",):
+        np.save(os.path.join(out_dir, f"{prefix}_cpl_{f}.npy"), cpls[f][idx].astype(np.float64))
 
 
 def peaks():
@@ -511,7 +536,7 @@ def run_ours(args, rank, world, local):
     timer = lib.Timer()
     out = {}
 
-    def resident_leg(io_blocks, pattern, sg, nq, per_q, steps, warmup, check, target=0):
+    def resident_leg(io_blocks, pattern, sg, nq, per_q, steps, warmup, check, target=0, dump=None):
         n = nq * per_q
         t = traces.uniform_trace(n, NUM_BLOCKS, io_blocks=io_blocks, pattern=pattern, sg=sg, seed=plan["trace_seed"],
                                  target=target)
@@ -546,6 +571,8 @@ def run_ours(args, rank, world, local):
         assert (c["status"] == 0).all() and (c["resid"] == 0).all() and (c["used_len"] > 0).all(), "bad completions"
         if check:
             check(t, arena)
+        if dump and args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, dump, t, arena, c, torch)
         del arena, d_reqs, d_iovs, d_cpls
         torch.cuda.empty_cache()
         return n, ms, launches, t
@@ -574,7 +601,8 @@ def run_ours(args, rank, world, local):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    n, ms, launches, _ = resident_leg(8, "randread", "single", nq, per_q, args.steps, args.warmup, check_randread)
+    n, ms, launches, _ = resident_leg(8, "randread", "single", nq, per_q, args.steps, args.warmup, check_randread,
+                                      dump="rand4k")
     iops = aggregate(n, args.steps, world, ms)
     per_launch_ms = ms / max(1, launches)
     achieved = 2 * 4096 * n / (per_launch_ms / 1e3) / 1e9
@@ -1000,7 +1028,7 @@ def vhost_user_leg(args, device: int, mode: str, queue_counts=(64,), gpus=None, 
     ring = 1024
     max_q = max(queue_counts)
     nb = 1 << 21                                         # 1 GiB bdev: far larger than L2
-    tmp = tempfile.mkdtemp(prefix="oimvu")
+    tmp = tempfile.mkdtemp(prefix="oimvu", dir="/tmp")        # socket paths must fit sun_path (108 bytes)
     os.mkdir(os.path.join(tmp, "vhost"))
     rpc = os.path.join(tmp, "rpc.sock")
     log = open(os.path.join(tmp, "daemon.log"), "wb")

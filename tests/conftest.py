@@ -21,6 +21,18 @@ def oracles():
     return bindings
 
 
+@pytest.fixture()
+def sock_dir():
+    """A fresh directory for Unix domain sockets, removed afterwards.  A socket's path must fit sun_path
+    (108 bytes), which a path under pytest's tmp_path does not when TMPDIR is deep, so it lives under /tmp."""
+    import pathlib
+    import shutil
+    import tempfile
+    d = tempfile.mkdtemp(prefix="oim-", dir="/tmp")
+    yield pathlib.Path(d)
+    shutil.rmtree(d, ignore_errors=True)
+
+
 @pytest.fixture(scope="session")
 def gpu():
     """liboimgpu.so initialised on cuda:0.  Fails loudly when the extension is missing."""

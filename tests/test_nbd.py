@@ -15,6 +15,7 @@ import time
 import numpy as np
 import pytest
 
+import util
 from oim_b200 import traces
 
 NB, BS = 8192, 512                     # 4 MiB
@@ -148,14 +149,36 @@ def tails():
     return {"disc": encode((DISC, 0, 0, b""), 0xD15C), "garbage": b"\x00" * 28}
 
 
+def reference_replies(oracles, key, ops, tail):
+    """run_reference as stored: every reply (length, 8-byte digest, first 16 bytes) and the store's SHA-256"""
+    def produce():
+        out, store = run_reference(oracles, ops, tail)
+        return {"len": [len(r) for r in out], "digest": np.array([util.digest64(r) for r in out], np.uint64),
+                "head": np.array([np.frombuffer(r[:16].ljust(16, b"\0"), np.uint8) for r in out]), "store_sha": util.sha(store)}
+    return util.reference("nbd_reference", key, produce)
+
+
+def assert_replies_equal(ops, got, want):
+    assert len(got) == len(want["len"])
+    for i, g in enumerate(got):
+        w = (int(want["len"][i]), int(want["digest"][i]))
+        assert (len(g), util.digest64(g)) == w, \
+            f"reply {i} to {ops[i][:3] if i < len(ops) else 'tail'} differs: {g[:24]!r} vs {bytes(want['head'][i])!r}..."
+
+
 def test_reference_nbd_loop_known_answers(oracles):
-    """the harness against the reference alone: known answers, so that the GPU test below compares against
+    """the harness against the reference alone: known answers, so that the tests below compare against
     something that is itself pinned"""
-    if not oracles.ref_available():
-        pytest.skip("oracle/_ref not built here")
     ops = [(WRITE, 4096, 1024, b"\xab" * 1024), (READ, 4096, 1024, b""), (READ, 4096 + 7, 512, b""), (TRIM, 4096, 512, b""),
            (READ, 4096, 1024, b""), (9, 0, 0, b""), (FLUSH, 0, 0, b"")]
-    out, store = run_reference(oracles, ops, tails()["disc"])
+
+    def produce():
+        out, store = run_reference(oracles, ops, tails()["disc"])
+        return {"replies": np.frombuffer(b"".join(out), np.uint8), "len": [len(r) for r in out], "store": store[4096:5120]}
+    z = util.reference("nbd_known_answers", "disc", produce)
+    out = [bytes(r) for r in np.split(z["replies"], np.cumsum(z["len"])[:-1])]
+    store = np.zeros(8192, np.uint8)
+    store[4096:5120] = z["store"]
 
     def rep(h, err):
         return struct.pack(">II8s", REP_MAGIC, err, struct.pack("<Q", 0x1000 + h))
@@ -196,17 +219,13 @@ def run_restatement(oracles, ops, tail):
 
 @pytest.mark.parametrize("seed", range(8))
 def test_nbd_restatement_matches_reference(oracles, seed):
-    if not oracles.ref_available():
-        pytest.skip("oracle/_ref not built here")
     ops = script(seed)
     tail = tails()["disc" if seed % 2 == 0 else "garbage"]
-    want, want_store = run_reference(oracles, ops, tail)
+    want = reference_replies(oracles, f"seed{seed}", ops, tail)
     got, got_store, rc = run_restatement(oracles, ops, tail)
     assert rc == (0 if seed % 2 == 0 else -22)
-    assert len(got) == len(want)
-    for i, (g, w) in enumerate(zip(got, want)):
-        assert g == w, f"reply {i} to {ops[i][:3] if i < len(ops) else 'tail'} differs: {g[:24]!r} vs {w[:24]!r}"
-    assert (got_store == want_store).all()
+    assert_replies_equal(ops, got, want)
+    assert util.sha(got_store) == str(want["store_sha"])
     assert any(op[0] == TRIM and op[2] == 0 for s in range(8) for op in script(s)), "the zero-length TRIM case is in the scripts"
 
 
@@ -215,10 +234,7 @@ def test_nbd_restatement_matches_reference(oracles, seed):
 def test_cuda_nbd_matches_reference(gpu, oracles, seed):
     ops = script(seed)
     tail = tails()["disc" if seed % 2 == 0 else "garbage"]
-    if oracles.ref_available():
-        want, want_store = run_reference(oracles, ops, tail)
-    else:
-        want, want_store, _ = run_restatement(oracles, ops, tail)
+    want = reference_replies(oracles, f"seed{seed}", ops, tail)
     name = f"nbd{seed}"
     gpu.construct_malloc_bdev(NB, BS, name=name, device=0)
     try:
@@ -236,13 +252,11 @@ def test_cuda_nbd_matches_reference(gpu, oracles, seed):
         assert not th.is_alive()
         a.close()
         assert rc == [0 if seed % 2 == 0 else -22]
-        assert len(got) == len(want)
-        for i, (g, w) in enumerate(zip(got, want)):
-            assert g == w, f"reply {i} to {ops[i][:3] if i < len(ops) else 'tail'} differs: {g[:24]!r} vs {w[:24]!r}"
-        assert (gpu.bdev_read_raw(name, 0, NB * BS) == want_store).all()
+        assert_replies_equal(ops, got, want)
+        assert util.sha(gpu.bdev_read_raw(name, 0, NB * BS)) == str(want["store_sha"])
         st = gpu.get_bdevs_iostat(name)
-        ok_reads = sum(1 for op, r in zip(ops, want) if op[0] == READ and r[4:8] == b"\x00" * 4)
-        ok_writes = sum(1 for op, r in zip(ops, want) if op[0] == WRITE and r[4:8] == b"\x00" * 4)
+        ok_reads = sum(1 for op, r in zip(ops, want["head"]) if op[0] == READ and not r[4:8].any())
+        ok_writes = sum(1 for op, r in zip(ops, want["head"]) if op[0] == WRITE and not r[4:8].any())
         assert (st["num_read_ops"], st["num_write_ops"]) == (ok_reads, ok_writes)
     finally:
         gpu.delete_bdev(name)

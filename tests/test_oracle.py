@@ -1,5 +1,6 @@
 """Pin the CPU checkers: restatement (oracle/oim_oracle.c) vs the compiled reference
-(oracle/_ref, built from /root/reference) vs the committed golden vectors.  CPU only."""
+(oracle/_ref, built from the original project's sources; its results stored under tests/golden/reference)
+vs the committed golden vectors.  CPU only."""
 import glob
 import os
 
@@ -43,14 +44,12 @@ def test_restatement_matches_golden_vectors(oracles, path):
 
 @pytest.mark.parametrize("seed", range(200, 212))
 def test_restatement_matches_reference_on_fresh_fuzz(oracles, seed):
-    if not oracles.ref_available():
-        pytest.skip("oracle/_ref not built here (no /root/reference)")
     nb = 32768
     t = traces.fuzz_trace(300, nb, seed=seed, max_io_blocks=[8, 64, 300][seed % 3])
-    want = util.run_oracle(oracles.RefOracle, t, nb)
+    want = util.reference_run("fresh_fuzz", f"seed{seed}", t, nb)
     got = util.run_oracle(oracles.PortOracle, t, nb)
-    util.assert_cpls_equal(got[0], want[0], t.reqs, f"seed {seed}")
-    assert (got[1] == want[1]).all() and (got[2] == want[2]).all()
+    util.assert_cpls_equal(got[0], want["cpls"], t.reqs, f"seed {seed}")
+    assert util.sha(got[1]) == str(want["arena_sha"]) and util.sha(got[2]) == str(want["store_sha"])
 
 
 # ---- known-answer cases of the reference's own unit tests ------------------------------------
@@ -64,9 +63,7 @@ def _one(o, cdb, direction, iovs):
 @pytest.mark.parametrize("which", ["port", "ref"])
 def test_scsi_bdev_ut_lba_range_and_xfer_len(oracles, which):
     """S/test/unit/lib/scsi/scsi_bdev.c/scsi_bdev_ut.c:639-794 (lba_range_test, xfer_len_test)"""
-    if which == "ref" and not oracles.ref_available():
-        pytest.skip("no oracle/_ref")
-    cls = oracles.RefOracle if which == "ref" else oracles.PortOracle
+    cls = util.stored_reference("lba_range_and_xfer_len") if which == "ref" else oracles.PortOracle
     buf = np.zeros(5 * 512, dtype=np.uint8)
     with cls(4) as o:                                   # "Test block device size of 4 blocks"
         c = _one(o, abi.cdb_rw(abi.READ_16, 0, 1), abi.DIR_FROM_DEV, [(buf.ctypes.data, 512)])
@@ -94,9 +91,7 @@ def test_scsi_bdev_ut_lba_range_and_xfer_len(oracles, which):
 @pytest.mark.parametrize("which", ["port", "ref"])
 def test_scsi_bdev_ut_xfer(oracles, which):
     """scsi_bdev_ut.c:796-897 (_xfer_test): READ16, WRITE16, UNMAP with 2 descriptors, SYNC16"""
-    if which == "ref" and not oracles.ref_available():
-        pytest.skip("no oracle/_ref")
-    cls = oracles.RefOracle if which == "ref" else oracles.PortOracle
+    cls = util.stored_reference("xfer", keep_store=True) if which == "ref" else oracles.PortOracle
     with cls(2048) as o:
         o.store[:] = 0xEE
         buf = np.full(512, 0xA3, dtype=np.uint8)
@@ -116,18 +111,24 @@ def test_scsi_bdev_ut_xfer(oracles, which):
 def test_vhost_ut_desc_to_iov(oracles, which):
     """S/test/unit/lib/vhost/vhost.c/vhost_ut.c:188-262: GPA->VVA and the 2 MiB / region split rule"""
     import ctypes as C
-    if which == "ref" and not oracles.ref_available():
-        pytest.skip("no oracle/_ref")
-    path, prefix = (oracles.REF_SO, "oimref") if which == "ref" else (oracles.PORT_SO, "oimorc")
-    fn = getattr(C.CDLL(path), prefix + "_desc_to_iov")
-    fn.restype = C.c_int
-    fn.argtypes = [C.c_void_p, C.c_uint32, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint32]
+    import itertools
     regions = np.array([0, 0x400000, 0x1000000, 0x400000, 0x400000, 0x2000000], dtype=np.uint64)
+    calls = itertools.count()
 
-    def conv(addr, length, start=0):
+    def run(path, prefix, addr, length, start):
+        fn = getattr(C.CDLL(path), prefix + "_desc_to_iov")
+        fn.restype = C.c_int
+        fn.argtypes = [C.c_void_p, C.c_uint32, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint32]
         out = np.zeros(4, dtype=abi.iov_dtype)
         n = fn(regions.ctypes.data, 2, addr, length, out.ctypes.data, start)
         return n, [(int(a), int(l)) for a, l in zip(out["addr"][:max(n, 0)], out["len"][:max(n, 0)])]
+
+    def conv(addr, length, start=0):
+        if which == "port":
+            return run(oracles.PORT_SO, "oimorc", addr, length, start)
+        n, iov = util.reference_json("known_answers", f"desc_to_iov.{next(calls)}",
+                                     lambda: run(oracles.REF_SO, "oimref", addr, length, start))
+        return n, [tuple(x) for x in iov]
 
     assert conv(0x110000, 0x1000) == (1, [(0x1110000, 0x1000)])
     assert conv(0x110000, 0x1000, abi.IOVS_MAX - 1) == (1, [(0x1110000, 0x1000)])
@@ -173,9 +174,7 @@ class HostBuf:
 
 @pytest.mark.parametrize("which", ["port", "ref"])
 def test_bdevio_suite(oracles, which):
-    if which == "ref" and not oracles.ref_available():
-        pytest.skip("no oracle/_ref")
-    cls = oracles.RefOracle if which == "ref" else oracles.PortOracle
+    cls = util.stored_reference("bdevio") if which == "ref" else oracles.PortOracle
     nb = 65536        # 32 MiB, as S/test/bdev/bdev.conf.in:5-7
     with cls(nb) as o:
         run_bdevio(o.submit, HostBuf, nb)

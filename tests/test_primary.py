@@ -24,9 +24,7 @@ def _one(o, cdb, n):
 @pytest.mark.parametrize("which", ["port", "ref"])
 def test_inquiry_known_answers(oracles, which):
     """what a Linux guest sees (pkg/oim-controller/controller_test.go:336-338 asserts vendor 'INTEL   ')"""
-    if which == "ref" and not oracles.ref_available():
-        pytest.skip("no oracle/_ref")
-    cls = oracles.RefOracle if which == "ref" else oracles.PortOracle
+    cls = util.stored_reference("inquiry") if which == "ref" else oracles.PortOracle
     with cls(NB, name=NAME) as o:
         c, d = _one(o, [0x12, 0, 0, 0, 96], 96)
         assert c["status"] == 0 and c["resid"] == 0
@@ -48,15 +46,17 @@ def test_inquiry_known_answers(oracles, which):
 
 @pytest.mark.parametrize("seed", range(500, 508))
 def test_primary_restatement_matches_reference(oracles, seed):
-    if not oracles.ref_available():
-        pytest.skip("oracle/_ref not built here")
     t = traces.primary_trace(300, seed=seed)
-    with oracles.RefOracle(NB, name=NAME) as probe:
-        dev_id = probe.scsi_dev_id
-    want = util.run_oracle(oracles.RefOracle, t, NB, name=NAME)
-    got = util.run_oracle(oracles.PortOracle, t, NB, name=NAME, scsi_dev_id=dev_id)
-    util.assert_cpls_equal(got[0], want[0], t.reqs, f"seed {seed}")
-    assert (got[1] == want[1]).all()
+
+    def produce():
+        with oracles.RefOracle(NB, name=NAME) as probe:
+            dev_id = probe.scsi_dev_id
+        cpls, arena, _ = util.run_oracle(oracles.RefOracle, t, NB, name=NAME)
+        return {"cpls": cpls, "arena_sha": util.sha(arena), "scsi_dev_id": dev_id}
+    want = util.reference("primary_commands", f"seed{seed}", produce)
+    got = util.run_oracle(oracles.PortOracle, t, NB, name=NAME, scsi_dev_id=int(want["scsi_dev_id"]))
+    util.assert_cpls_equal(got[0], want["cpls"], t.reqs, f"seed {seed}")
+    assert util.sha(got[1]) == str(want["arena_sha"])
 
 
 def test_primary_golden_fixture(oracles):

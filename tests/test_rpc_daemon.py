@@ -1,7 +1,7 @@
 """Boundary B1 (SURVEY.md 8(b)): the JSON-RPC wire behaviour of oim-gpu-vhost, compared reply by reply
 with the REFERENCE'S OWN server (S/lib/jsonrpc + S/lib/rpc + the registered bdev / vhost handlers,
-compiled into oracle/_ref and polled in-process) and with the expectations of OIM's Go tests
-(pkg/spdk/spdk_test.go:36-331, pkg/oim-controller/controller_test.go:226-304).
+compiled into oracle/_ref; its replies stored in tests/golden/reference/rpc_transcripts.json.xz) and with the
+expectations of OIM's Go tests (pkg/spdk/spdk_test.go:36-331, pkg/oim-controller/controller_test.go:226-304).
 
 CPU: the daemon runs with --control-only (bookkeeping only, no data path exists in that mode).
 GPU: the real daemon, plus a data check through the same process-external socket."""
@@ -15,6 +15,8 @@ import sys
 import time
 
 import pytest
+
+import util
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DAEMON = os.environ.get("OIM_DAEMON_PATH") or os.path.join(ROOT, "oim_b200", "oim-gpu-vhost")   # override: sanitizer builds
@@ -69,29 +71,57 @@ def norm(reply: bytes) -> str:
     return re.sub(r'"uuid":"(?!11111111-)[0-9a-f-]{36}"', '"uuid":"<uuid>"', s)     # random unless the test chose it
 
 
+class Transcript:
+    """The reference server's side of a test's conversation, as stored by util.reference_json: every request the test
+    sent and the reference's reply, with the vhost socket directory written as <vdir>.  In record mode the requests go
+    to the live reference server (`live`) and the transcript is written down."""
+
+    def __init__(self, key: str, vdir: str, live: Client | None = None):
+        self.key, self.vdir, self.live = key, vdir, live
+        self.log = [] if live else util.reference_json("rpc_transcripts", key, None)
+        self.pos = self.id = 0
+
+    def raw(self, data: bytes, expect_reply=True, timeout=5.0) -> bytes:
+        req = data.decode().replace(self.vdir, "<vdir>")
+        if self.live:
+            reply = self.live.raw(data, expect_reply, timeout)
+            self.log.append([req, reply.decode().replace(self.vdir, "<vdir>")])
+            return reply
+        assert self.pos < len(self.log), f"{self.key}: the stored transcript ends before {req!r}"
+        want, reply = self.log[self.pos]
+        self.pos += 1
+        assert req == want, f"{self.key}: the test sent {req!r} where the stored transcript has {want!r}"
+        return reply.replace("<vdir>", self.vdir).encode()
+
+    call = Client.call
+
+
 @pytest.fixture()
-def servers(oracles, tmp_path):
-    """(ours, reference) clients on two fresh servers sharing one vhost socket directory name"""
-    if not oracles.ref_available():
-        pytest.skip("oracle/_ref not built here")
+def servers(oracles, sock_dir, request):
+    """(ours, reference) clients sharing one vhost socket directory name: ours on a fresh server, the reference's
+    replies from its stored transcript (recorded on a fresh reference server)"""
     from oim_b200 import build
     build.build()
-    vdir = tmp_path / "vhost"
+    vdir = sock_dir / "vhost"
     vdir.mkdir()
-    ours_sock, ref_sock = str(tmp_path / "ours.sock"), str(tmp_path / "ref.sock")
+    ours_sock, ref_sock = str(sock_dir / "ours.sock"), str(sock_dir / "ref.sock")
     mode = [] if os.environ.get("OIM_RPC_TEST_GPU") else ["--control-only"]
-    proc = subprocess.Popen([DAEMON, "-r", ours_sock, "-S", str(vdir), *mode], stderr=subprocess.PIPE)
-    # the reference server in a process of its own, so every test starts from SPDK's boot state
-    refp = subprocess.Popen([sys.executable, os.path.join(ROOT, "tests", "ref_rpc_server.py"), ref_sock, str(vdir)],
-                            stderr=subprocess.PIPE)
+    procs = [subprocess.Popen([DAEMON, "-r", ours_sock, "-S", str(vdir), *mode], stderr=subprocess.PIPE)]
+    if util.RECORD:
+        # the reference server in a process of its own, so every test starts from SPDK's boot state
+        procs.append(subprocess.Popen([sys.executable, os.path.join(ROOT, "tests", "ref_rpc_server.py"), ref_sock, str(vdir)],
+                                      stderr=subprocess.PIPE))
     for _ in range(500):
-        if os.path.exists(ours_sock) and os.path.exists(ref_sock):
+        if os.path.exists(ours_sock) and (not util.RECORD or os.path.exists(ref_sock)):
             break
         time.sleep(0.01)
+    ref = Transcript(request.node.name, str(vdir), Client(ref_sock) if util.RECORD else None)
     try:
-        yield Client(ours_sock), Client(ref_sock), str(vdir)
+        yield Client(ours_sock), ref, str(vdir)
+        if util.RECORD:
+            util.reference_json("rpc_transcripts", ref.key, lambda: ref.log)
     finally:
-        for p in (proc, refp):
+        for p in procs:
             p.terminate()
             p.wait(5)
 
@@ -262,15 +292,15 @@ def test_map_unmap_volume_sequence(servers):
 
 
 @pytest.mark.gpu
-def test_daemon_on_gpu_config1(tmp_path):
+def test_daemon_on_gpu_config1(sock_dir):
     """BASELINE config 1: 'Malloc bdev 64 MiB via oim-controller MapVolume' against the real daemon
     (HBM-backed stores): ProvisionMallocBDev -> MapVolume -> get -> UnmapVolume, plus the RBD-shaped volume
     of config 3 (construct_rbd_bdev as pkg/oim-controller/controller.go:284-295 issues it)."""
     from oim_b200 import build
     build.build()
-    vdir = tmp_path / "vhost"
+    vdir = sock_dir / "vhost"
     vdir.mkdir()
-    sock = str(tmp_path / "rpc.sock")
+    sock = str(sock_dir / "rpc.sock")
     proc = subprocess.Popen([DAEMON, "-r", sock, "-S", str(vdir), "-s", "256", "-R", "--gpus", "0", "--rbd-size", str(1 << 30)],
                             stderr=subprocess.PIPE)
     try:
@@ -350,7 +380,7 @@ def test_rpc_random_call_sequences(servers):
             both(servers, "delete_bdev", {"name": b["name"]})
 
 
-def test_config_dump_and_restore(tmp_path):
+def test_config_dump_and_restore(sock_dir):
     """get_subsystems / get_subsystem_config + tools/oimcfg.py: the {method, params} lists of
     spdk_bdev_subsystem_config_json (S/lib/bdev/bdev.c:676-708; bdev_malloc.c:350-368, bdev_rbd.c:635-666) and
     spdk_vhost_config_json (S/lib/vhost/vhost.c:1460-1494; vhost_scsi.c:1459-1499), replayed into a fresh daemon"""
@@ -360,7 +390,7 @@ def test_config_dump_and_restore(tmp_path):
     import oimcfg
 
     def daemon(tag):
-        d = tmp_path / tag
+        d = sock_dir / tag
         d.mkdir()
         (d / "vhost").mkdir()
         p = subprocess.Popen([DAEMON, "-r", str(d / "rpc.sock"), "-S", str(d / "vhost"), "--control-only"], stderr=subprocess.PIPE)

@@ -3,7 +3,8 @@
 
 The same master script (oim_b200/vhost_user_master.py) runs against oim-gpu-vhost and against the REFERENCE'S OWN
 transport + vhost-scsi + bdev stack (oracle/_ref/liboim_ref_vhost.so: S/lib/vhost/rte_vhost/* compiled where it
-lies), and the protocol transcripts and the guest memory are compared.
+lies), and the protocol transcripts and the guest memory are compared.  The reference's side is stored
+(tests/golden/reference/vhost_user.json.xz: transcripts, completions, digests of the guest memory; see tests/util.py).
 
 CPU: handshake, control queue, event queue / hot-plug (our daemon with --control-only: no data path exists then).
 GPU: request queues served by the kernel, launch-per-kick and resident-poller mode."""
@@ -16,6 +17,7 @@ import time
 import numpy as np
 import pytest
 
+import util
 from oim_b200 import abi, traces, vring
 from test_rpc_daemon import DAEMON, ROOT, Client
 from oim_b200 import vhost_user_master as vu
@@ -249,15 +251,14 @@ def used_set(mem, ring, n):
 
 
 @pytest.fixture()
-def slaves(oracles, tmp_path):
-    if not oracles.ref_available() or not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "liboim_ref_vhost.so")):
-        pytest.skip("oracle/_ref/liboim_ref_vhost.so not built here")
+def slaves(oracles, sock_dir):
     from oim_b200 import build
     build.build()
     made = []
 
     def make(kind, extra=()):
-        s = Slave(kind, tmp_path, extra)
+        assert kind == "ours" or util.RECORD, "the reference slave runs only to record its side (util.reference_json)"
+        s = Slave(kind, sock_dir, extra)
         made.append(s)
         provision(s)
         return s
@@ -268,13 +269,38 @@ def slaves(oracles, tmp_path):
         print(open(s.dir / "log.txt", errors="replace").read()[-3000:])
 
 
+def reference_side(slaves, key: str, run):
+    """what `run(reference slave)` returned, as stored (util.reference_json); in record mode from a live reference
+    slave (the reference's own transport + vhost-scsi + bdev stack, oracle/_ref/liboim_ref_vhost.so)"""
+    return util.reference_json("vhost_user", key, lambda: run(slaves("ref")))
+
+
+def transcript(log):
+    """a master's transcript back from its stored form (JSON lists)"""
+    return tuple(log) if log and log[0] == "dropped" else [tuple(e) for e in log]
+
+
+def assert_same_memory(got: np.ndarray, want, what="guest memory"):
+    util.assert_same_digests(got, np.array(want, dtype=np.uint64), what)
+
+
+def skip_without_gpu_after_recording():
+    import torch
+    if util.RECORD and not torch.cuda.is_available():
+        pytest.skip("the reference's side is recorded; our side needs a GPU")
+
+
 def test_vhost_user_handshake_control_and_event_queues(slaves):
-    ours, ref = slaves("ours", ["--control-only"]), slaves("ref")
+    ours = slaves("ours", ["--control-only"])
     lo, so, img, rings = run_script(ours, [], data=False)
-    lr, sr, _, _ = run_script(ref, [], data=False)
+
+    def ref_run(ref):
+        lr, sr, _, _ = run_script(ref, [], data=False)
+        return {"log": lr, "mem": util.block_digests(mask(sr["end"], img, rings)).tolist(), "used_cq": used_set(sr["end"], rings[0], 8)}
+    r = reference_side(slaves, "handshake", ref_run)
+    lr = transcript(r["log"])
     assert deliberate(lo) == deliberate(lr), f"protocol transcripts differ:\nours {lo}\nref  {lr}"
-    a, b = mask(so["end"], img, rings), mask(sr["end"], img, rings)
-    assert (a == b).all(), f"guest memory differs at {np.nonzero(a != b)[0][:16]}"
+    assert_same_memory(mask(so["end"], img, rings), r["mem"])
     # and the values themselves, so that two equally wrong slaves cannot pass
     d = dict((k, v) for k, v in lo if v is not None)
     assert d[vu.GET_FEATURES] == 0x150000007 and d[vu.GET_PROTOCOL_FEATURES] == 0x21D and d[vu.GET_QUEUE_NUM] == 128
@@ -283,7 +309,7 @@ def test_vhost_user_handshake_control_and_event_queues(slaves):
     cq, eq, _ = rings
     resp = [int(so["end"][cq[3] + 64 * k + 32]) for k in range(8)]
     assert resp[:4] == [0, 2, 3, 3] and int(so["end"][cq[3] + 64 * 4 + 36]) == 2 and resp[6] == 0xEE
-    assert used_set(so["end"], cq, 8) == used_set(sr["end"], cq, 8) == [(0, 0), (2, 1), (4, 1), (6, 1), (8, 1), (10, 0), (12, 1), (14, 0)]
+    assert used_set(so["end"], cq, 8) == [tuple(u) for u in r["used_cq"]] == [(0, 0), (2, 1), (4, 1), (6, 1), (8, 1), (10, 0), (12, 1), (14, 0)]
     ev = so["end"][eq[3]:eq[3] + 16].tobytes()
     assert struct.unpack("<I8sI", ev) == (1, bytes([1, 1, 0, 0, 0, 0, 0, 0]), 1)      # TRANSPORT_RESET, target 1, RESCAN
     ev2 = so["end"][eq[3] + 32:eq[3] + 48].tobytes()
@@ -293,14 +319,12 @@ def test_vhost_user_handshake_control_and_event_queues(slaves):
 def test_remove_controller_with_a_master_connected_is_busy(slaves):
     """spdk_vhost_dev_unregister: "Controller %s has still valid connection" -> -EBUSY (S/lib/vhost/vhost.c:783-788); round 1
     tore the session down instead (ADVICE r1).  Same RPC replies from both servers, before and after the master leaves."""
-    ours, ref = slaves("ours", ["--control-only"]), slaves("ref")
-    for s in (ours, ref):
+    def run(s):
         for t in range(8):
             s.call("remove_vhost_scsi_target", {"ctrlr": "scsi0", "scsi_target_num": t})     # whatever provision() attached
         m = vu.Master(s.sock("scsi0"))
         m.get_u64(vu.GET_FEATURES)                       # the connection is established and served
         busy = s.call("remove_vhost_controller", {"ctrlr": "scsi0"})
-        assert b'"code":-32602' in busy and b"Device or resource busy" in busy, (s.kind, busy)
         m.close()
         deadline = time.time() + 10
         while True:                                      # the slave notices the closed socket on its own thread
@@ -308,8 +332,12 @@ def test_remove_controller_with_a_master_connected_is_busy(slaves):
             if b'"result":true' in r or time.time() > deadline:
                 break
             time.sleep(0.05)
-        assert b'"result":true' in r, (s.kind, r)
-        assert not os.path.exists(s.sock("scsi0"))
+        return {"busy": busy.decode(), "last": r.decode(), "socket_left": os.path.exists(s.sock("scsi0"))}
+    got = run(slaves("ours", ["--control-only"]))
+    for kind, out in (("ours", got), ("ref", reference_side(slaves, "remove_busy_controller", run))):
+        assert '"code":-32602' in out["busy"] and "Device or resource busy" in out["busy"], (kind, out)
+        assert '"result":true' in out["last"], (kind, out)
+        assert not out["socket_left"], kind
 
 
 def test_vhost_user_reconnect_and_odd_masters(slaves):
@@ -352,24 +380,31 @@ def test_cuda_vhost_user_io_matches_reference(slaves, mode):
         if torch.cuda.device_count() < 2:
             pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
         extra += ["--gpus", "0,1"]
-    ours, ref = slaves("ours", extra), slaves("ref")
+    import json
+    import re
     rq = make_requests(11)
+
+    def iostat(s):
+        """get_bdevs_iostat: what each bdev served, counted the way the bdev layer counts (the sessions are gone by
+        now: the counters outlive them)"""
+        time.sleep(0.5)
+        return json.loads(re.sub(rb'"(tick_rate|\w+_latency_ticks)":\d+', rb'"\1":0', s.call("get_bdevs_iostat")))["result"]
+
+    def ref_run(ref):
+        lr, sr, img, rings = run_script(ref, rq, data=True)
+        return {"log": lr, "mem": util.block_digests(mask(sr["end"], img, rings)).tolist(), "iostat": iostat(ref)}
+    r = reference_side(slaves, "io", ref_run)                # the reference's side is the same for every mode
+    skip_without_gpu_after_recording()
+    ours = slaves("ours", extra)
     lo, so, img, rings = run_script(ours, rq, data=True)
-    lr, sr, _, _ = run_script(ref, rq, data=True)
+    lr = transcript(r["log"])
     assert deliberate(lo) == deliberate(lr), f"protocol transcripts differ:\nours {lo}\nref  {lr}"
-    a, b = mask(so["end"], img, rings), mask(sr["end"], img, rings)
-    assert (a == b).all(), f"guest memory differs at {np.nonzero(a != b)[0][:16]}"
+    assert_same_memory(mask(so["end"], img, rings), r["mem"])
     assert dict((k, v) for k, v in lo if v is not None)[vu.GET_VRING_BASE] is not None
     # the READ on queue 3 went to the hot-plugged target (a fresh Malloc bdev: zeros)
     data_off = META_END - 4 * 8192
     assert (so["end"][data_off:data_off + 4096] == 0).all()
-    # get_bdevs_iostat: what each bdev served, counted the way the bdev layer counts (the sessions are gone by
-    # now: the counters outlive them)
-    import json
-    import re
-    time.sleep(0.5)
-    a = json.loads(re.sub(rb'"(tick_rate|\w+_latency_ticks)":\d+', rb'"\1":0', ours.call("get_bdevs_iostat")))["result"]
-    b = json.loads(re.sub(rb'"(tick_rate|\w+_latency_ticks)":\d+', rb'"\1":0', ref.call("get_bdevs_iostat")))["result"]
+    a, b = iostat(ours), r["iostat"]
     assert a == b, f"iostat differs:\nours {a}\nref  {b}"
     raw = [x for x in json.loads(ours.call("get_bdevs_iostat"))["result"] if x.get("name") == "M0"][0]
     assert raw["read_latency_ticks"] > 0 and raw["write_latency_ticks"] > 0, raw      # summed by the mover warps, 1 GHz ticks
@@ -430,10 +465,14 @@ def two_vm_script(s: Slave):
 @pytest.mark.gpu
 @pytest.mark.parametrize("mode", ["kick", "poller"])
 def test_cuda_vhost_user_sessions_come_and_go(slaves, mode):
-    ours, ref = slaves("ours", ["--poller"] if mode == "poller" else []), slaves("ref")
-    got, want = two_vm_script(ours), two_vm_script(ref)
+    def ref_run(ref):
+        out = two_vm_script(ref)
+        return {**{k: util.block_digests(out[k]).tolist() for k in ("a", "b", "c")}, "a_base": out["a_base"], "c_base": out["c_base"]}
+    want = reference_side(slaves, "sessions", ref_run)         # the reference's side is the same for both modes
+    skip_without_gpu_after_recording()
+    got = two_vm_script(slaves("ours", ["--poller"] if mode == "poller" else []))
     for k in ("a", "b", "c"):
-        assert (got[k] == want[k]).all(), f"VM {k}: guest memory differs at {np.nonzero(got[k] != want[k])[0][:16]}"
+        assert_same_memory(got[k], want[k], f"VM {k}: guest memory")
     assert got["a_base"] == want["a_base"] and got["c_base"] == want["c_base"]
     assert got["a_base"][2] == 64 - 0 or got["a_base"][2] > 0
 
@@ -505,11 +544,9 @@ def fuzz_script(m: vu.Master, ram: vu.GuestRam, rng, nmsg=60):
 
 def test_vhost_user_random_message_sequences(slaves):
     """differential fuzzing of the protocol state machine: same random sequences, same replies"""
-    ours, ref = slaves("ours", ["--control-only"]), slaves("ref")
-    agree = 0
-    for seed in range(150):
+    def run(s):
         logs = []
-        for s in (ours, ref):
+        for seed in range(150):
             ram = vu.GuestRam(4 << 20)
             m = vu.Master(s.sock("scsi0"))
             try:
@@ -521,9 +558,12 @@ def test_vhost_user_random_message_sequences(slaves):
                 m.close()
                 ram.close()
             assert s.p.poll() is None, f"seed {seed}: the {s.kind} server died"
-        assert deliberate(logs[0]) == deliberate(logs[1]), f"seed {seed}: transcripts differ\nours {logs[0]}\nref  {logs[1]}"
-        agree += 1
-    assert agree == 150
+        return logs
+    got = run(slaves("ours", ["--control-only"]))
+    want = [transcript(x) for x in reference_side(slaves, "random_message_sequences", run)]
+    assert len(got) == len(want) == 150
+    for seed, (a, b) in enumerate(zip(got, want)):
+        assert deliberate(a) == deliberate(b), f"seed {seed}: transcripts differ\nours {a}\nref  {b}"
 
 
 def random_control_requests(ram, img, ring, rng):
@@ -590,12 +630,19 @@ def control_fuzz_script(s: Slave, seed: int):
 
 
 def test_vhost_user_control_queue_fuzz(slaves):
-    ours, ref = slaves("ours", ["--control-only"]), slaves("ref")
+    def ref_run(ref):
+        out = []
+        for seed in range(12):
+            mem, used = control_fuzz_script(ref, seed)
+            out.append({"mem": util.block_digests(mem).tolist(), "used": used})
+        return out
+    want = reference_side(slaves, "control_queue_fuzz", ref_run)
+    ours = slaves("ours", ["--control-only"])
     for seed in range(12):
         a, ua = control_fuzz_script(ours, seed)
-        b, ub = control_fuzz_script(ref, seed)
+        ub = [tuple(u) for u in want[seed]["used"]]
         assert ua == ub, f"seed {seed}: used elements differ\nours {ua}\nref  {ub}"
-        assert (a == b).all(), f"seed {seed}: guest memory differs at {np.nonzero(a != b)[0][:16]}"
+        assert_same_memory(a, want[seed]["mem"], f"seed {seed}: guest memory")
 
 
 def test_vhost_user_many_masters_and_hot_plug_at_once(slaves):

@@ -3,6 +3,7 @@ CPU: the C restatement against the compiled reference.  GPU: the kernel's own ri
 import numpy as np
 import pytest
 
+import util
 from oim_b200 import traces, vring
 
 
@@ -31,18 +32,26 @@ def run_kicks_oracle(cls, rq, nb, ring_size, seed, mutate=True, contiguous=False
 
 @pytest.mark.parametrize("seed", range(400, 412))
 def test_vring_restatement_matches_reference(oracles, seed):
-    if not oracles.ref_available():
-        pytest.skip("oracle/_ref not built here")
     nb, rq = 32768, make_requests(seed)
     ring = [64, 256, 1024][seed % 3]
-    want, want_store = run_kicks_oracle(oracles.RefOracle, rq, nb, ring, seed)
+
+    def produce():
+        kicks, store = run_kicks_oracle(oracles.RefOracle, rq, nb, ring, seed)
+        mem = [util.block_digests(m) for m, _, _ in kicks]
+        return {"mem": np.concatenate(mem), "mem_count": np.array([len(m) for m in mem]),
+                "cursors": np.array([c for _, _, c in kicks]),
+                "used": np.array([u for _, used, _ in kicks for u in used], dtype=np.int64).reshape(-1, 2),
+                "used_count": np.array([len(used) for _, used, _ in kicks]), "store_sha": util.sha(store)}
+    want = util.reference("vring_kicks", f"seed{seed}", produce)
     got, got_store = run_kicks_oracle(oracles.PortOracle, rq, nb, ring, seed)
-    assert len(got) == len(want)
-    for k, (g, w) in enumerate(zip(got, want)):
-        assert g[2] == w[2], f"kick {k}: cursors"
-        assert g[1] == w[1], f"kick {k}: used elements"
-        assert (g[0] == w[0]).all(), f"kick {k}: guest memory differs at {np.nonzero(g[0] != w[0])[0][:8]}"
-    assert (got_store == want_store).all()
+    assert len(got) == len(want["cursors"])
+    used = np.split(want["used"], np.cumsum(want["used_count"])[:-1])
+    mem = np.split(want["mem"], np.cumsum(want["mem_count"])[:-1])
+    for k, (g, c, u, m) in enumerate(zip(got, want["cursors"], used, mem)):
+        assert g[2] == tuple(int(x) for x in c), f"kick {k}: cursors"
+        assert g[1] == [tuple(int(x) for x in e) for e in u], f"kick {k}: used elements"
+        util.assert_same_digests(g[0], m, f"kick {k}: guest memory")
+    assert util.sha(got_store) == str(want["store_sha"])
 
 
 def test_vring_broken_avail_index(oracles):
